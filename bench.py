@@ -4,9 +4,10 @@ metric : env-steps/sec over collect+update (the reference's ``train_speed``, fsr
 step   : ONE collect + update cycle (trainer.train_step + policy_update_fn)
 configs: --config c1 | c2 (default, the headline) | c3 | c4 | c5   (BASELINE.json "configs", in order)
 
-  python bench.py [--config c2] [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--config c2] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
-Prints one JSON line (rank 0).  See DESIGN.md "Measurement" for how every field is derived.
+Prints one JSON line (rank 0).  See DESIGN.md "Measurement" for how every field is derived.  --dump-outputs writes what
+the last timed step computed as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -276,12 +277,14 @@ def run_ours(args):
     collect_s = 0.0
     for _ in range(args.steps):
         c0 = col.collect_time
-        one_cycle(trainer)
+        stats = one_cycle(trainer)
         collect_s += col.collect_time - c0
     ev1.record()
     torch.cuda.synchronize()
     launches = int(_fl.lib.fsrl_launch_count()) - launches0
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, agent.policy, stats, buf)
     if dist is not None:
         t = torch.tensor([ms], device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -376,6 +379,32 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 1 << 16                 # replay rows sampled for --dump-outputs
+DUMP_LIMIT = 64 << 20               # bytes
+
+
+def dump_outputs(out_dir, policy, stats, buf):
+    """What a caller of the timed path holds after its last step, as float32 / float64 arrays: the collect statistics
+    (collect_*), the update's per-step losses (update_*), the Lagrange multipliers, every network parameter (params)
+    and the replay rows the collect wrote (buffer_*; a fixed, seeded sample of DUMP_ROWS rows, the same in every run)."""
+    arrays = {"collect_" + k: np.float64(v) for k, v in stats.items()}
+    for k, v in policy.last_stats.items():
+        v = np.asarray(v)
+        arrays["update_" + k] = v if v.dtype == np.float32 else v.astype(np.float64)
+    if hasattr(policy, "lagrangians"):
+        arrays["lagrangians"] = np.asarray(policy.lagrangians(), np.float64)
+    arrays["params"] = policy.arena.theta.detach().float().cpu().numpy()
+    rows = np.random.default_rng(0).choice(buf.maxsize, min(DUMP_ROWS, buf.maxsize), replace=False)
+    rows = torch.from_numpy(np.sort(rows)).to(buf.device)
+    for k in ("obs", "obs_next", "act", "rew", "cost", "logp", "terminated", "truncated"):
+        arrays["buffer_" + k] = getattr(buf, k)[rows].float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name.replace("/", "_") + ".npy"), a)
+
+
 def other_roofline(cfg, agent, steps_per_cycle, ms_cycle, collect_s, pk, how):
     """CPO: Fisher/Hessian-vector products dominate (~ 4 x 2 N P flops each, SURVEY.md 8d); SAC: latency of a gradient step."""
     s0 = agent.policy.arena.slots[0]
@@ -401,13 +430,16 @@ def other_roofline(cfg, agent, steps_per_cycle, ms_cycle, collect_s, pk, how):
 # -------------------------------------------------------------------------------------------------
 # reference arm / cpu_baseline: the reference's own classes on the host cores (oracle/refarm.py)
 # -------------------------------------------------------------------------------------------------
+REF_MISSING = "oracle/_ref is missing: __graft_entry__.build() installs it where a checkout of liuzuxin/FSRL is present (FSRL_REFERENCE)"
+
+
 def _reference_dir():
-    d = os.path.join(ROOT, "baseline", "_ref")
-    return d if os.path.isdir(os.path.join(d, "fsrl")) else None
+    from oracle.refarm import REF_DIR
+    return REF_DIR if os.path.isdir(os.path.join(REF_DIR, "fsrl")) else None
 
 
 def cpu_reference(config="c2", sample_envs=32, cycles=1, threads=None, runner=None):
-    """One or more collect+update cycles of the UNMODIFIED reference (baseline/_ref): fsrl.data.FastCollector over one worker
+    """One or more collect+update cycles of the UNMODIFIED reference (oracle/_ref): fsrl.data.FastCollector over one worker
     PROCESS per env (tianshou SubprocVectorEnv protocol; the simulator inside a worker is the numpy twin of the device env
     model, pybullet / mujoco being absent), fsrl.policy.PPOLagrangian.process_fn + learn.  c1 runs verbatim (4 envs); the other
     PPO configs run their network / batch shapes on a bounded sample of `sample_envs` envs (one process per env does not
@@ -418,7 +450,7 @@ def cpu_reference(config="c2", sample_envs=32, cycles=1, threads=None, runner=No
         return cpu_port_other(cfg, sample_envs)
     ref_dir = _reference_dir()
     if ref_dir is None:
-        raise SystemExit("baseline/_ref is missing: run __graft_entry__.build() in the build container first")
+        return {"value": None, "unit": "env-steps/s", "kind": "reference", "unavailable": REF_MISSING}
     from oracle import refarm
     n_env = cfg["envs"] if config == "c1" else min(sample_envs, cfg["envs"])
     threads = threads or 4                                        # the reference's default (ppol_cfg.py:11 thread = 4)
@@ -436,7 +468,7 @@ def cpu_reference(config="c2", sample_envs=32, cycles=1, threads=None, runner=No
             "torch_threads": threads, "kind": "reference", "collect_s": tc, "update_s": tu,
             "same_config": config == "c1",
             "sample": f"{n_env} envs x {runner.T} steps x {cycles} cycle(s), {cfg['hidden'][0]}-wide MLPs, batch {cfg['batch']}, "
-                      f"repeat {cfg['repeat']}: unmodified fsrl.data.FastCollector + fsrl.policy.PPOLagrangian from baseline/_ref "
+                      f"repeat {cfg['repeat']}: unmodified fsrl.data.FastCollector + fsrl.policy.PPOLagrangian from oracle/_ref "
                       f"(no fsrl_b200 import), one env worker process per env, torch.set_num_threads({threads}) (reference default); "
                       f"collect {tc:.1f} s + update {tu:.1f} s"}
 
@@ -460,7 +492,7 @@ def run_reference(args):
     from oracle import refarm
     ref_dir = _reference_dir()
     if ref_dir is None:
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref missing (build() installs it)"}))
+        print(json.dumps({"impl": "reference", "unavailable": REF_MISSING}))
         return
     n_env = cfg["envs"] if args.config == "c1" else min(args.cpu_envs, cfg["envs"])
     threads = 4
@@ -499,6 +531,8 @@ if __name__ == "__main__":
     ap.add_argument("--cpu-envs", type=int, default=32,
                     help="envs (= worker processes) of the bounded CPU sample for configs other than c1")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     a = ap.parse_args()
     if a.impl == "reference":
         run_reference(a)

@@ -807,7 +807,7 @@ def _save(name, cases):
 
 
 def check(ref_dir, rtol=2e-5):
-    """Re-run the PPO cases with the reference found in `ref_dir` (e.g. the baseline/_ref install) and
+    """Re-run the PPO cases with the reference found in `ref_dir` (e.g. the oracle/_ref install) and
     compare with the committed fixture: the installed copy must behave like the source tree."""
     global REF
     REF = ref_dir

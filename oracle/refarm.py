@@ -1,5 +1,5 @@
-"""The CPU arm of bench.py (test / baseline infrastructure): the UNMODIFIED reference classes from ``baseline/_ref``
-(``pip install --no-deps --target``; ``/root/reference`` in the build container) run the whole collect + update
+"""The CPU arm of bench.py (test / baseline infrastructure): the UNMODIFIED reference classes from ``oracle/_ref``
+(``install()``: ``pip install --no-deps --target`` from a checkout of liuzuxin/FSRL) run the whole collect + update
 cycle on the host cores --
 
 * ``fsrl.data.FastCollector.collect`` (fast_collector.py:192-408) drives a vector env whose every env lives in its
@@ -14,14 +14,35 @@ from __future__ import annotations
 
 import multiprocessing as mp
 import os
+import shutil
+import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+# the checkout of liuzuxin/FSRL the install is made from; FSRL_REFERENCE names another one
+REF_SRC = os.environ.get("FSRL_REFERENCE", "/root/reference")
 _REF = None
+
+
+def install(src: str = REF_SRC, dst: str = REF_DIR) -> None:
+    """Install the reference package from the checkout ``src`` into ``dst`` unless it is there already or ``src``
+    holds no checkout.  No dependencies are installed: ``bootstrap`` supplies the third-party packages from
+    oracle/shims.  pip writes build files beside the sources, so it builds from a copy and ``src`` may be read-only."""
+    if os.path.isdir(os.path.join(dst, "fsrl")) or not os.path.isdir(os.path.join(src, "fsrl")):
+        return
+    with tempfile.TemporaryDirectory() as tmp:
+        work = os.path.join(tmp, "reference")
+        shutil.copytree(src, work, ignore=shutil.ignore_patterns(".git"), copy_function=shutil.copyfile)
+        for d, _, _ in os.walk(work):
+            os.chmod(d, 0o755)                  # copytree keeps the directories' modes, and pip writes into them
+        subprocess.check_call([sys.executable, "-m", "pip", "install", "--quiet", "--no-index", "--no-build-isolation",
+                               "--no-deps", "--no-cache-dir", "--target", dst, work])
 
 
 def bootstrap(ref_dir: str):

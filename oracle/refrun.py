@@ -7,9 +7,8 @@ code is involved), puts ``ref_dir`` first on ``sys.path`` so that ``import fsrl`
 and adds the one missing tianshou method the learners call, ``Batch.split`` (restated in
 oracle/ppo.py::split_indices, SURVEY.md 2.3 [UNVERIFIED]).
 
-ref_dir is ``/root/reference`` in the build container (golden-vector generation) or
-``baseline/_ref`` (``pip install --no-deps --target``, travels to the GPU box) for
-``bench.py --impl reference`` / ``cpu_baseline``.
+ref_dir is a checkout of the reference (golden-vector generation) or ``oracle/_ref``
+(``refarm.install``: ``pip install --no-deps --target``) for ``bench.py --impl reference`` / ``cpu_baseline``.
 """
 from __future__ import annotations
 

@@ -1,7 +1,7 @@
 """CPU-only stand-ins for the third-party packages the reference (liuzuxin/FSRL) imports and that are absent
 here: ``tianshou`` (setup.py:16, ~=0.5.0), ``gymnasium``, ``bullet_safety_gym``, ``safety_gymnasium``, ``pyrallis``,
 ``h5py``.  Test / baseline infrastructure: ``install()`` lets ``import fsrl`` resolve to the UNMODIFIED reference
-package (``/root/reference`` in the build container, ``baseline/_ref`` on the GPU box) in a process that never
+package (a checkout of it, or its install under ``oracle/_ref``) in a process that never
 imports ``fsrl_b200`` -- so the reference arm of bench.py maps no product code.
 
 Only what ``fsrl`` touches on the measured path is provided (SURVEY.md 2.3, Appendix C [UNVERIFIED restatements of

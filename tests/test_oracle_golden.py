@@ -383,15 +383,15 @@ def test_nstep_glue_replays_reference_compute_nstep_returns(golden_dir):
 
 
 def test_installed_reference_reproduces_golden():
-    """baseline/_ref (the --no-deps pip install used by `bench.py --impl reference`) runs through the same
+    """oracle/_ref (the --no-deps pip install used by `bench.py --impl reference`) runs through the same
     shims and reproduces the committed PPO fixture.  Runs in a subprocess: loading the reference rewires
     sys.modules (tianshou / gymnasium shims, `fsrl` = the reference)."""
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref = os.path.join(root, "baseline", "_ref")
+    ref = os.path.join(root, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref, "fsrl")):
-        pytest.skip("baseline/_ref not built (python -c 'import __graft_entry__ as g; g.build()')")
+        pytest.skip("oracle/_ref not installed (build() installs it where a checkout of liuzuxin/FSRL is present)")
     out = subprocess.run([sys.executable, os.path.join(root, "oracle", "make_golden_policies.py"), "--check", ref],
                          capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]

@@ -210,9 +210,6 @@ SIGNATURES = {
     "fsrl_ppo_persist_ws_floats": (c_size, [c_int, c_int, c_int]),
     "fsrl_ppo_persist_p2p_floats": (c_size, [c_int]),
     "fsrl_ppo_persist_active": (c_int, [ctypes.POINTER(PpoUpdate), ctypes.c_longlong, c_int]),
-    "fsrl_debug_clocks": (c_int, [ctypes.POINTER(ctypes.c_longlong)]),
-    "fsrl_debug_cta_cycles": (c_int, [ctypes.POINTER(ctypes.c_longlong)]),
-    "fsrl_ppo_phase_times": (c_int, [ctypes.POINTER(PpoUpdate), c_int, c_int, ctypes.POINTER(c_f32), c_vp]),
     "fsrl_ppo_lag_epoch": (c_int, [ctypes.POINTER(PpoUpdate), ctypes.c_longlong, c_int, c_int,
                                    ctypes.c_longlong, ctypes.POINTER(c_int), c_vp]),
 }

@@ -220,8 +220,9 @@ cpo_rfwd_kernel(const fsrl_engine_t e, const fsrl_netref_t np_, const fsrl_netre
     const int r0 = blockIdx.x * TT::R;
     const int inp = TT::in_pad(D);
     // tangent parameter views
-    const float* v_w1t = pv; const float* v_b1 = v_w1t + (size_t)D * H; const float* v_w2t = v_b1 + H;
-    const float* v_b2 = v_w2t + (size_t)H * H; const float* v_w3t = v_b2 + H; const float* v_b3 = v_w3t + (size_t)H * out;
+    const NetLayout L(D, H, out, np_.n_extra);
+    const float* v_w1t = pv + L.w1; const float* v_b1 = pv + L.b1; const float* v_w2t = pv + L.w2;
+    const float* v_b2 = pv + L.b2; const float* v_w3t = pv + L.w3; const float* v_b3 = pv + L.b3;
     float* xs = smem;                                   // [R][inp]
     float* ta = xs + (size_t)TT::R * inp;               // tile A [R][LDA]  (Rh1, later h2 cache)
     float* tb = ta + (size_t)TT::R * TT::LDA;           // tile B           (h1 cache, later Rh2)
@@ -305,7 +306,7 @@ cpo_rbwd_kernel(const fsrl_engine_t e, const fsrl_netref_t np_, const fsrl_netre
     const int D = np_.D, out = np_.out;
     const int tid = threadIdx.x;
     const int r0 = blockIdx.x * TT::R;
-    const float* v_w3t = pv + (size_t)D * H + H + (size_t)H * H + H;
+    const float* v_w3t = pv + NetLayout(D, H, out, np_.n_extra).w3;
     float* ta = smem;                                   // Rda2 tile
     float* tb = ta + (size_t)TT::R * TT::LDA;           // da2 (primal) tile
     float* wst = tb + (size_t)TT::R * TT::LDA;
@@ -375,16 +376,6 @@ __global__ void vec_add_scaled_kernel(const float* a, float s, const float* b, f
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = a[i] + s * b[i];
 }
-// mirror of the W2 block of a tangent vector: dst[o][k] = src[k][o]
-__global__ void vec_w2_mirror_kernel(const float* src_w2t, float* dst, int H) {
-    __shared__ float tile[32][33];
-    const int tt = blockIdx.x;
-    const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
-    const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
-    for (int q = 0; q < 4; ++q) tile[ly + 8 * q][lx] = src_w2t[(size_t)(k0 + ly + 8 * q) * H + o0 + lx];
-    __syncthreads();
-    for (int q = 0; q < 4; ++q) dst[(size_t)(o0 + ly + 8 * q) * H + k0 + lx] = tile[lx][ly + 8 * q];
-}
 
 }  // namespace fsrl
 
@@ -437,11 +428,15 @@ extern "C" int fsrl_cpo_hvp(const fsrl_cpo_t* d, const float* v, float* v_w2n_sc
     const fsrl_netref_t& nr_ = d->actor_r.nets[0];
     const int H = np_.H, D = np_.D, out = np_.out;
     const int B = (int)d->N;
-    const long long P = (long long)D * H + H + (long long)H * H + H + (long long)H * out + out + np_.n_extra;
+    const NetLayout L(D, H, out, np_.n_extra);
+    const long long P = L.size;
     fsrl_eng_input_t in;
     in.xa = d->obs; in.ia = d->perm; in.xb = nullptr; in.ib = nullptr; in.Da = D; in.Db = 0;
-    vec_w2_mirror_kernel<<<(H / 32) * (H / 32), 256, 0, s>>>(v + (size_t)D * H + H, v_w2n_scratch, H);
-    FSRL_LAUNCH_CHECK();
+    W2Mirrors vm = {};   // mirror of the tangent vector's W2 block
+    vm.w2t[0] = v + L.w2;
+    vm.w2n[0] = v_w2n_scratch;
+    rc = w2_mirror(vm, 1, H, s);
+    if (rc) return rc;
     ENG_DISPATCH_H(H, {
         using TT = MlpTile<HH>;
         const size_t smf = sizeof(float) * ((size_t)TT::R * TT::in_pad(D) + 2 * (size_t)TT::R * TT::LDA + TT::stage_floats() + 2 * (size_t)HH * out);
@@ -456,7 +451,7 @@ extern "C" int fsrl_cpo_hvp(const fsrl_cpo_t* d, const float* v, float* v_w2n_sc
         float* r_out = sc + 4 * (size_t)d->eng.bmax * H;
         float* r_dout = r_out + (size_t)d->eng.bmax * 16;
         (void)Rv;
-        cpo_rhead_kernel<<<(unsigned)((d->N + 255) / 256), 256, 0, s>>>(*d, d->N, r_out, v + (P - np_.n_extra), r_dout);
+        cpo_rhead_kernel<<<(unsigned)((d->N + 255) / 256), 256, 0, s>>>(*d, d->N, r_out, v + L.extra, r_dout);
         FSRL_LAUNCH_CHECK();
     }
     ENG_DISPATCH_H(H, {

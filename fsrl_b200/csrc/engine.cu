@@ -158,12 +158,7 @@ eng_wgrad_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, const fsrl_eng_
     const long long row_lo = (long long)blockIdx.z * rows_per;
     const int B = (int)((row_lo >= Btot) ? 0 : ((Btot - row_lo < rows_per) ? (Btot - row_lo) : rows_per));
     if (B == 0) return;
-    if (roles.dst) {
-        float* g = roles.dst;
-        size_t o = 0;
-        nv.g_w1t = g + o; o += (size_t)nr.D * H; nv.g_b1 = g + o; o += H; nv.g_w2t = g + o; o += (size_t)H * H;
-        nv.g_b2 = g + o; o += H; nv.g_w3t = g + o; o += (size_t)H * nr.out; nv.g_b3 = g + o; o += nr.out; nv.g_extra = g + o;
-    }
+    if (roles.dst) eng_grad_view(nv, roles.dst, NetLayout(nr.D, H, nr.out, nr.n_extra));
     nv.s_h1 = const_cast<float*>(roles.L2 ? roles.L2 : nv.s_h1) + (size_t)row_lo * H;
     nv.s_dz2 = const_cast<float*>(roles.G2 ? roles.G2 : nv.s_dz2) + (size_t)row_lo * H;
     nv.s_dz1 = const_cast<float*>(roles.G1 ? roles.G1 : nv.s_dz1) + (size_t)row_lo * H;
@@ -368,39 +363,31 @@ eng_wgrad_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, const fsrl_eng_
 // ---------------------------------------------------------------------------------------------
 // Adam over a set of nets (torch.optim.Adam arithmetic), optional L2 term, W2 mirror upkeep
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ float eng_adam_one(float p, float g, float& m, float& v, float w1, float b2,
-                                              float w2, float bc2s, float eps, float neg_step) {
-    m = m + w1 * (g - m);
-    v = v * b2 + (w2 * g) * g;
-    const float denom = sqrtf(v) / bc2s + eps;
-    return p + (neg_step * m) / denom;
-}
-
 __global__ void __launch_bounds__(256)
-eng_adam_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, float w1, float b2, float w2, float bc2s,
-                float eps, float neg_step, float gscale, float l2x2, const float* norm_sq, float max_norm) {
+eng_adam_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, const AdamStep ad, float gscale, float l2x2,
+                const float* norm_sq, float max_norm) {
     __shared__ float tile[32][33];
     const fsrl_netref_t nr = nl.nets[blockIdx.y];
     const int H = nr.H;
     float scale = gscale;
     if (norm_sq && max_norm > 0.f) scale *= fminf(max_norm / (sqrtf(*norm_sq) + 1e-6f), 1.0f);
-    const long long w2s = (long long)nr.D * H + H;          // start of the W2 block inside the net
-    const long long n_total = w2s + (long long)H * H + H + (long long)H * nr.out + nr.out + nr.n_extra;
-    const int n_plain_blocks = (int)((n_total + 255) / 256);
+    const NetLayout L(nr);
+    const int n_plain_blocks = (int)((L.size + 255) / 256);
     if ((int)blockIdx.x < n_plain_blocks) {
         const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
-        if (j >= n_total || (j >= w2s && j < w2s + (long long)H * H)) return;
+        if (j >= L.size || (j >= L.w2 && j < L.b2)) return;
         const long long i = nr.off + j;
         float m = e.adam_m[i], v = e.adam_v[i];
         const float p = e.theta[i];
         const float g = e.grad[i] * scale + l2x2 * p;
-        e.theta[i] = eng_adam_one(p, g, m, v, w1, b2, w2, bc2s, eps, neg_step);
+        e.theta[i] = adam_one(p, g, m, v, ad);
         e.adam_m[i] = m; e.adam_v[i] = v;
     } else {
         const int tt = blockIdx.x - n_plain_blocks;
         if (tt >= (H / 32) * (H / 32)) return;
-        const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
-        const long long base = nr.off + w2s;
+        int k0, o0;
+        w2_tile_origin(tt, H, k0, o0);
+        const long long base = nr.off + L.w2;
         const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
@@ -409,17 +396,11 @@ eng_adam_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, float w1, float 
             float m = e.adam_m[i], v = e.adam_v[i];
             float p = e.theta[i];
             const float g = e.grad[i] * scale + l2x2 * p;
-            p = eng_adam_one(p, g, m, v, w1, b2, w2, bc2s, eps, neg_step);
+            p = adam_one(p, g, m, v, ad);
             e.theta[i] = p; e.adam_m[i] = m; e.adam_v[i] = v;
             tile[kk][lx] = p;
         }
-        __syncthreads();
-        float* mir = e.w2n + nr.w2n_off;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int oo = ly + 8 * q;
-            mir[(size_t)(o0 + oo) * H + k0 + lx] = tile[lx][oo];
-        }
+        w2_tile_store_mirror(tile, e.w2n + nr.w2n_off, H, k0, o0);
     }
 }
 
@@ -430,49 +411,45 @@ eng_polyak_kernel(const fsrl_engine_t e, const fsrl_netlist_t dst, const fsrl_ne
     __shared__ float tile[32][33];
     const fsrl_netref_t nd = dst.nets[blockIdx.y], ns = src.nets[blockIdx.y];
     const int H = nd.H;
-    const long long w2s = (long long)nd.D * H + H;
-    const long long n_total = w2s + (long long)H * H + H + (long long)H * nd.out + nd.out + nd.n_extra;
-    const int n_plain_blocks = (int)((n_total + 255) / 256);
+    const NetLayout L(nd);
+    const int n_plain_blocks = (int)((L.size + 255) / 256);
     if ((int)blockIdx.x < n_plain_blocks) {
         const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
-        if (j >= n_total || (j >= w2s && j < w2s + (long long)H * H)) return;
+        if (j >= L.size || (j >= L.w2 && j < L.b2)) return;
         e.theta[nd.off + j] = tau * e.theta[ns.off + j] + (1.0f - tau) * e.theta[nd.off + j];
     } else {
         const int tt = blockIdx.x - n_plain_blocks;
         if (tt >= (H / 32) * (H / 32)) return;
-        const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
+        int k0, o0;
+        w2_tile_origin(tt, H, k0, o0);
         const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int kk = ly + 8 * q;
-            const long long j = w2s + (long long)(k0 + kk) * H + o0 + lx;
+            const long long j = L.w2 + (long long)(k0 + kk) * H + o0 + lx;
             const float p = tau * e.theta[ns.off + j] + (1.0f - tau) * e.theta[nd.off + j];
             e.theta[nd.off + j] = p;
             tile[kk][lx] = p;
         }
-        __syncthreads();
-        float* mir = e.w2n + nd.w2n_off;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int oo = ly + 8 * q;
-            mir[(size_t)(o0 + oo) * H + k0 + lx] = tile[lx][oo];
-        }
+        w2_tile_store_mirror(tile, e.w2n + nd.w2n_off, H, k0, o0);
     }
 }
 
-__global__ void eng_mirror_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl) {
+__global__ void __launch_bounds__(256) w2_mirror_kernel(const __grid_constant__ W2Mirrors mr, int H) {
     __shared__ float tile[32][33];
-    const fsrl_netref_t nr = nl.nets[blockIdx.y];
-    const int H = nr.H;
-    const int tt = blockIdx.x;
-    if (tt >= (H / 32) * (H / 32)) return;
-    const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
-    const float* src = e.theta + nr.off + (long long)nr.D * H + H;
+    int k0, o0;
+    w2_tile_origin(blockIdx.x, H, k0, o0);
+    const float* src = mr.w2t[blockIdx.y];
     const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
+#pragma unroll
     for (int q = 0; q < 4; ++q) tile[ly + 8 * q][lx] = src[(size_t)(k0 + ly + 8 * q) * H + o0 + lx];
-    __syncthreads();
-    float* mir = e.w2n + nr.w2n_off;
-    for (int q = 0; q < 4; ++q) mir[(size_t)(o0 + ly + 8 * q) * H + k0 + lx] = tile[lx][ly + 8 * q];
+    w2_tile_store_mirror(tile, mr.w2n[blockIdx.y], H, k0, o0);
+}
+
+int w2_mirror(const W2Mirrors& m, int n, int H, cudaStream_t s) {
+    w2_mirror_kernel<<<dim3((H / 32) * (H / 32), n), 256, 0, s>>>(m, H);
+    FSRL_LAUNCH_CHECK();
+    return FSRL_OK;
 }
 
 static int eng_check(const fsrl_engine_t* e, const fsrl_netlist_t* nl) {
@@ -487,6 +464,17 @@ static int eng_check(const fsrl_engine_t* e, const fsrl_netlist_t* nl) {
         FSRL_REQUIRE(nl->nets[i].D >= 1 && nl->nets[i].D <= FSRL_ENG_DX_LD, "engine: input dim %d unsupported", nl->nets[i].D);
     }
     return FSRL_OK;
+}
+
+// largest parameter count of the listed nets (grid size of the per-net element kernels)
+static long long max_net_size(const fsrl_netlist_t* nl) {
+    long long maxn = 0;
+    for (int i = 0; i < nl->n; ++i) {
+        const fsrl_netref_t& n = nl->nets[i];
+        const long long tot = NetLayout(n).size;
+        if (tot > maxn) maxn = tot;
+    }
+    return maxn;
 }
 
 }  // namespace fsrl
@@ -534,7 +522,7 @@ namespace fsrl {
 // zero the gradient range of the listed nets (needed before a split-K wgrad that does not accumulate)
 __global__ void eng_zero_grad_kernel(const fsrl_engine_t e, const fsrl_netlist_t nl, float* dst_override) {
     const fsrl_netref_t nr = nl.nets[blockIdx.y];
-    const long long n = (long long)nr.D * nr.H + nr.H + (long long)nr.H * nr.H + nr.H + (long long)nr.H * nr.out + nr.out + nr.n_extra;
+    const long long n = NetLayout(nr).size;
     float* g = dst_override ? dst_override : e.grad + nr.off;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) g[i] = 0.f;
 }
@@ -581,18 +569,12 @@ extern "C" int fsrl_engine_adam(const fsrl_engine_t* e, const fsrl_netlist_t* nl
     FSRL_REQUIRE(e->adam_m && e->adam_v && step >= 1, "engine_adam: missing moments or step < 1");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
-    long long maxn = 0;
-    int H = nl->nets[0].H;
-    for (int i = 0; i < nl->n; ++i) {
-        const fsrl_netref_t& n = nl->nets[i];
-        const long long tot = (long long)n.D * H + H + (long long)H * H + H + (long long)H * n.out + n.out + n.n_extra;
-        if (tot > maxn) maxn = tot;
-    }
-    const int blocks = (int)((maxn + 255) / 256) + (H / 32) * (H / 32);
-    eng_adam_kernel<<<dim3(blocks, nl->n), 256, 0, s>>>(*e, *nl, (float)(1.0 - beta1), (float)beta2,
-                                                        (float)(1.0 - beta2), (float)sqrt(bc2), (float)eps,
-                                                        (float)(-(lr / bc1)), (float)grad_scale,
-                                                        (float)(2.0 * l2_reg), norm_sq, (float)max_grad_norm);
+    const int H = nl->nets[0].H;
+    const int blocks = (int)((max_net_size(nl) + 255) / 256) + (H / 32) * (H / 32);
+    const AdamStep ad = {(float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), (float)sqrt(bc2), (float)eps,
+                         (float)(-(lr / bc1))};
+    eng_adam_kernel<<<dim3(blocks, nl->n), 256, 0, s>>>(*e, *nl, ad, (float)grad_scale, (float)(2.0 * l2_reg), norm_sq,
+                                                        (float)max_grad_norm);
     FSRL_LAUNCH_CHECK();
     return FSRL_OK;
 }
@@ -605,15 +587,12 @@ extern "C" int fsrl_engine_polyak(const fsrl_engine_t* e, const fsrl_netlist_t* 
     if (rc) return rc;
     FSRL_REQUIRE(dst->n == src->n, "polyak: net lists differ in length");
     FSRL_REQUIRE(tau >= 0.0 && tau <= 1.0, "tau should be in [0, 1]");
-    long long maxn = 0;
     const int H = dst->nets[0].H;
     for (int i = 0; i < dst->n; ++i) {
         const fsrl_netref_t& n = dst->nets[i];
         FSRL_REQUIRE(n.D == src->nets[i].D && n.H == src->nets[i].H && n.out == src->nets[i].out, "polyak: shape mismatch");
-        const long long tot = (long long)n.D * H + H + (long long)H * H + H + (long long)H * n.out + n.out + n.n_extra;
-        if (tot > maxn) maxn = tot;
     }
-    const int blocks = (int)((maxn + 255) / 256) + (H / 32) * (H / 32);
+    const int blocks = (int)((max_net_size(dst) + 255) / 256) + (H / 32) * (H / 32);
     eng_polyak_kernel<<<dim3(blocks, dst->n), 256, 0, static_cast<cudaStream_t>(stream)>>>(*e, *dst, *src, (float)tau);
     FSRL_LAUNCH_CHECK();
     return FSRL_OK;
@@ -622,8 +601,11 @@ extern "C" int fsrl_engine_polyak(const fsrl_engine_t* e, const fsrl_netlist_t* 
 extern "C" int fsrl_engine_sync_mirror(const fsrl_engine_t* e, const fsrl_netlist_t* nl, void* stream) {
     int rc = eng_check(e, nl);
     if (rc) return rc;
-    const int H = nl->nets[0].H;
-    eng_mirror_kernel<<<dim3((H / 32) * (H / 32), nl->n), 256, 0, static_cast<cudaStream_t>(stream)>>>(*e, *nl);
-    FSRL_LAUNCH_CHECK();
-    return FSRL_OK;
+    W2Mirrors m = {};
+    for (int i = 0; i < nl->n; ++i) {
+        const fsrl_netref_t& n = nl->nets[i];
+        m.w2t[i] = e->theta + n.off + NetLayout(n).w2;
+        m.w2n[i] = e->w2n + n.w2n_off;
+    }
+    return w2_mirror(m, nl->n, nl->nets[0].H, static_cast<cudaStream_t>(stream));
 }

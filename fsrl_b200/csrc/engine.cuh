@@ -1,8 +1,8 @@
 // Shared declarations of the generic MLP engine (engine.cu) for the kernels built on top of it
 // (cpo.cu): scratch-slot views, input gathering, weight-gradient roles.
 #pragma once
+#include "arena.cuh"
 #include "mlp.cuh"
-#include "fsrl_b200.h"
 
 #define ENG_DISPATCH_H(Hv, ...)                                   \
     switch (Hv) {                                                 \
@@ -28,19 +28,20 @@ __host__ __device__ inline size_t eng_slot_floats(int H, int bmax) {
     return (size_t)bmax * (4 * (size_t)H + 2 * EDOUT_LD + FSRL_ENG_DX_LD);
 }
 
+// gradient pointers of a net whose gradient (layout L) starts at g
+__device__ __forceinline__ void eng_grad_view(EngView& v, float* g, const NetLayout& L) {
+    v.g_w1t = g + L.w1; v.g_b1 = g + L.b1; v.g_w2t = g + L.w2; v.g_b2 = g + L.b2;
+    v.g_w3t = g + L.w3; v.g_b3 = g + L.b3; v.g_extra = g + L.extra;
+}
+
 __device__ __forceinline__ EngView eng_view(const fsrl_engine_t& e, const fsrl_netref_t& n) {
     EngView v;
     const int H = n.H, D = n.D, out = n.out;
+    const NetLayout L(n);
     const float* th = e.theta + n.off;
-    float* g = e.grad + n.off;
-    size_t o = 0;
-    v.m.w1t = th + o; v.g_w1t = g + o; o += (size_t)D * H;
-    v.m.b1 = th + o;  v.g_b1 = g + o;  o += H;
-    v.m.w2t = th + o; v.g_w2t = g + o; o += (size_t)H * H;
-    v.m.b2 = th + o;  v.g_b2 = g + o;  o += H;
-    v.m.w3t = th + o; v.g_w3t = g + o; o += (size_t)H * out;
-    v.m.b3 = th + o;  v.g_b3 = g + o;  o += out;
-    v.g_extra = g + o;
+    v.m.w1t = th + L.w1; v.m.b1 = th + L.b1; v.m.w2t = th + L.w2;
+    v.m.b2 = th + L.b2;  v.m.w3t = th + L.w3; v.m.b3 = th + L.b3;
+    eng_grad_view(v, e.grad + n.off, L);
     v.m.in = D; v.m.H = H; v.m.out = out;
     v.w2n = e.w2n + n.w2n_off;
     float* sc = e.scratch + (size_t)n.slot * eng_slot_floats(H, e.bmax);

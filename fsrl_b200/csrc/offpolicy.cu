@@ -10,8 +10,7 @@
 //
 // One call runs `n_steps` complete gradient steps back to back (the loop of
 // OffpolicyTrainer.policy_update_fn, offpolicy.py:102-104) without returning to the host.
-#include "common.cuh"
-#include "fsrl_b200.h"
+#include "arena.cuh"
 
 namespace fsrl {
 
@@ -267,10 +266,6 @@ __global__ void alpha_step_kernel(const fsrl_offpolicy_t d, const float* __restr
     stat_out[FSRL_OFF_ST_ALPHA] = expf(nla);
 }
 
-static inline long long net_params(const fsrl_netref_t& r) {
-    return (long long)r.D * r.H + r.H + (long long)r.H * r.H + r.H + (long long)r.H * r.out + r.out + r.n_extra;
-}
-
 static inline fsrl_eng_input_t mk_in(const float* xa, const int* ia, int Da, const float* xb, const int* ib, int Db) {
     fsrl_eng_input_t in;
     in.xa = xa; in.ia = ia; in.xb = xb; in.ib = ib; in.Da = Da; in.Db = Db;
@@ -290,7 +285,7 @@ extern "C" int fsrl_allreduce_fused(void* comm, float* buf, long long n, void* s
 // data parallel: sum the gradient slices of a net list over the ranks (averaged by Adam's grad_scale)
 static int allreduce_grads(const fsrl_offpolicy_t* d, const fsrl_netlist_t* nl, void* stream) {
     long long offs[FSRL_ENG_MAX_NETS], counts[FSRL_ENG_MAX_NETS];
-    for (int i = 0; i < nl->n; ++i) { offs[i] = nl->nets[i].off; counts[i] = net_params(nl->nets[i]); }
+    for (int i = 0; i < nl->n; ++i) { offs[i] = nl->nets[i].off; counts[i] = NetLayout(nl->nets[i]).size; }
     return fsrl_allreduce_ranges(d->comm, d->eng.grad, offs, counts, nl->n, stream);
 }
 

@@ -22,10 +22,9 @@
 // Phase C (adam): clip scale + Adam over the flat parameter buffer; the W2 blocks are
 //   processed in 32x32 tiles through shared memory so that both the canonical W2t and its
 //   out-major mirror (needed by the backward GEMM) are written coalesced.
+#include "arena.cuh"
 #include "mlp.cuh"
-#include "fsrl_b200.h"
 #include "ppo_persist.cuh"
-#include <cstdlib>
 
 namespace fsrl {
 
@@ -33,18 +32,6 @@ constexpr int ST_ACTOR_REW = 0, ST_ACTOR_SAFETY = 1, ST_KL = 2, ST_VF0 = 3, ST_V
               ST_ENTROPY = 5, ST_GRADNORM = 6, ST_CLIPFRAC = 7;
 constexpr float LOG_SQRT_2PI_P = 0.9189385332046727f;
 constexpr int DOUT_LD = 16;   // scratch row stride of dOut (cols [A, 2A) carry dlog_sigma)
-
-__device__ long long g_dbg_clock[32];
-__device__ long long g_dbg_cta[512];
-#ifdef FSRL_DEBUG_CLOCKS   // per-phase clock64() stamps of CTA 0 (tools/kbench.py reads them back)
-#define DBG_T(i) do { if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 0) g_dbg_clock[i] = clock64(); } while (0)
-#define DBG_W(i) do { if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) g_dbg_clock[i] = clock64(); } while (0)
-#define DBG_CTA(i, v) do { if ((i) < 512) g_dbg_cta[i] = (v); } while (0)
-#else
-#define DBG_T(i) do { } while (0)
-#define DBG_W(i) do { } while (0)
-#define DBG_CTA(i, v) do { (void)(i); } while (0)
-#endif
 
 // Programmatic dependent launch (sm_90+): a kernel launched with the programmatic-serialization
 // attribute may start while its predecessor in the stream is still running; everything it reads
@@ -65,20 +52,25 @@ struct NetView {   // resolved pointers of one network inside the flat buffers
     float *s_h1, *s_h2, *s_dz1, *s_dz2, *s_dout;   // scratch [Bmax][H] / [Bmax][16]
 };
 
+// arena layout of net n: the actor (n = 0) heads actor_out columns and carries its log-sigma as extras
+__host__ __device__ __forceinline__ NetLayout ppo_layout(const fsrl_ppo_update_t& u, int n, int H) {
+    return NetLayout(u.D, H, (n == 0) ? u.actor_out : 1, (n == 0 && u.head_indep) ? u.A : 0);
+}
+
 __device__ __forceinline__ NetView net_view(const fsrl_ppo_update_t& u, int n) {
     NetView v;
     const int H = u.H, D = u.D;
     const int out = (n == 0) ? u.actor_out : 1;
+    const NetLayout L = ppo_layout(u, n, H);
     const float* th = u.theta + u.net_off[n];
     float* g = u.grad + u.net_off[n];
-    size_t o = 0;
-    v.m.w1t = th + o; v.g_w1t = g + o; o += (size_t)D * H;
-    v.m.b1 = th + o;  v.g_b1 = g + o;  o += H;
-    v.m.w2t = th + o; v.g_w2t = g + o; o += (size_t)H * H;
-    v.m.b2 = th + o;  v.g_b2 = g + o;  o += H;
-    v.m.w3t = th + o; v.g_w3t = g + o; o += (size_t)H * out;
-    v.m.b3 = th + o;  v.g_b3 = g + o;  o += out;
-    v.log_sigma = th + o; v.g_log_sigma = g + o;
+    v.m.w1t = th + L.w1; v.g_w1t = g + L.w1;
+    v.m.b1 = th + L.b1;  v.g_b1 = g + L.b1;
+    v.m.w2t = th + L.w2; v.g_w2t = g + L.w2;
+    v.m.b2 = th + L.b2;  v.g_b2 = g + L.b2;
+    v.m.w3t = th + L.w3; v.g_w3t = g + L.w3;
+    v.m.b3 = th + L.b3;  v.g_b3 = g + L.b3;
+    v.log_sigma = th + L.extra; v.g_log_sigma = g + L.extra;
     v.m.in = D; v.m.H = H; v.m.out = out;
     v.w2n = u.w2n + (size_t)n * H * H;
     float* sc = u.scratch + (size_t)n * u.bmax * (4 * (size_t)H + DOUT_LD);
@@ -126,22 +118,18 @@ ppo_fwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B) {
     float* xs = smem;                                   // [R][inp]
     float* h1 = xs + (size_t)TT::R * inp;               // [R][LDA]
     float* bs = h1 + (size_t)TT::R * TT::LDA;           // [H][SLAB_LDB]  (aliased by the reduce buffer)
-    DBG_T(16);
     // observations are constant during a repeat: loaded while the previous optimiser step drains
     for (int i = tid; i < TT::R * inp; i += MLP_TPB) {
         const int r = i / inp, k = i % inp;
         xs[i] = (r0 + r < B && k < D) ? u.obs[(size_t)row_of(u, mb_off, r0 + r) * D + k] : 0.f;
     }
-    DBG_T(17);
     pdl_wait();                                         // parameters of the previous step are final
     pdl_trigger();
     // bias of this thread's epilogue columns: requested now, consumed after the GEMM
     const float4 b2v = __ldg(reinterpret_cast<const float4*>(nv.m.b2 + c0 + (tid % (SLAB_NS / 4)) * 4));
-    DBG_T(18);
     if (net == 0 && slab == 0 && blockIdx.x == 0 && tid == 0) *u.norm_sq = 0.f;   // consumed by the previous step's Adam
     slab_load<H>(nv.m.w2t, H, c0, bs);                  // in flight during layer 1
     __syncthreads();
-    DBG_T(19);
     float c[TT::MT][TT::NT][4];
     tc_init_bias<H>(c, nv.m.b1);
     tc_gemm_direct<H>(c, xs, inp, D, nv.m.w1t);
@@ -150,17 +138,14 @@ ppo_fwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B) {
         *reinterpret_cast<float2*>(h1 + (size_t)row * TT::LDA + col) = h;
         if (slab == 0 && r0 + row < u.bmax) *reinterpret_cast<float2*>(nv.s_h1 + (size_t)(r0 + row) * H + col) = h;
     });
-    DBG_T(20);
     __pipeline_wait_prior(0);
     __syncthreads();
-    DBG_T(21);
     slab_gemm<H>(h1, TT::LDA, bs, bs, [&](int row, int c4, float4 v) {
         const float4 b = b2v;                           // c4 == (tid % 16) * 4 for every element this thread visits
         if (r0 + row < u.bmax)
             *reinterpret_cast<float4*>(nv.s_h2 + (size_t)(r0 + row) * H + c0 + c4) =
                 make_float4(fmaxf(v.x + b.x, 0.f), fmaxf(v.y + b.y, 0.f), fmaxf(v.z + b.z, 0.f), fmaxf(v.w + b.w, 0.f));
     });
-    DBG_T(22);
 }
 
 // per-row head dot product  out[j] = sum_k h2[k] * w3s[k][j]  over this lane's k subset, with the
@@ -199,7 +184,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
     float* w3s = bs + slab_buf_floats<H>();             // [H][out]
     float* sdout = w3s + (size_t)H * wout;              // [R][DOUT_LD]
     __shared__ float s_mean[2], s_rstd[2], s_b3[MLP_MAX_OUT], s_ls[8];
-    DBG_T(0);
     // everything that does not depend on the forward launch (weights, per-row loss inputs) is
     // requested before pdl_wait(): it overlaps the forward kernel's tail
     slab_load<H>(nv.w2n, H, c0, bs);                    // W2 in [out][in] layout: rows o, columns k-slab
@@ -223,7 +207,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
             if (u.value_clip) p_val = u.values[(size_t)(net - 1) * u.ld + id];
         }
     }
-    DBG_T(1);
     // per-minibatch advantage normalisation (ppo_lag.py:178-182): mean / 1/std of this minibatch
     // were computed for every minibatch of the repeat by ppo_adv_stats_kernel
     if (net == 0 && tid < u.C) {
@@ -244,8 +227,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
     __pipeline_commit();
     __pipeline_wait_prior(0);                            // slab (requested long ago) and h2 tile landed
     __syncthreads();
-
-    DBG_T(2);
     // ---- head forward (every slab CTA recomputes it: H x out MACs per row, negligible) -----------
     float out[MLP_MAX_OUT];
 #pragma unroll
@@ -267,8 +248,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
             out[j] = v + s_b3[j];
         }
     }
-
-    DBG_T(3);
     // ---- loss gradient at the head: one thread per row -----------------------------------------
     float st_a = 0.f, st_b = 0.f, st_c = 0.f, st_d = 0.f;     // per-thread stat partials
     if (part == 0) {
@@ -356,7 +335,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
                     make_float4(dd[j], dd[j + 1], dd[j + 2], dd[j + 3]);
         }
     }
-    DBG_T(4);
     // minibatch statistics (loss/actor_rew, actor_safety, kl, vf_i): warp-level partial sums and one
     // fire-and-forget reduction per warp -- no block barrier on the critical path
     if (slab == 0) {
@@ -378,8 +356,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
         }
     }
     __syncthreads();
-
-    DBG_T(5);
     // ---- backward through layer 3 and ReLU 2 (full width, redundant per slab: H x out per row) ----
     const int nout = (net == 0) ? u.A : 1;       // head columns that feed w3t (mu only)
     for (int e = tid; e < TT::R * (H / 4); e += MLP_TPB) {
@@ -396,10 +372,8 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
         *reinterpret_cast<float4*>(dz + (size_t)row * TT::LDA + k4) = g4;
         if (slab == 0 && r0 + row < u.bmax) *reinterpret_cast<float4*>(nv.s_dz2 + (size_t)(r0 + row) * H + k4) = g4;
     }
-    DBG_T(6);
     __pipeline_wait_prior(0);
     __syncthreads();
-    DBG_T(7);
     // the h2 tile is dead now: its space receives this slab's h1 columns (ReLU-1 mask of the epilogue)
     // while the GEMM runs (slab_gemm waits for outstanding async copies before its first barrier)
     for (int el = tid; el < TT::R * (SLAB_NS / 4); el += MLP_TPB) {
@@ -416,7 +390,6 @@ ppo_bwd_kernel(const fsrl_ppo_update_t u, int mb_off, int B, int slot) {
                 make_float4(hv.x > 0.f ? v.x : 0.f, hv.y > 0.f ? v.y : 0.f, hv.z > 0.f ? v.z : 0.f, hv.w > 0.f ? v.w : 0.f);
         }
     });
-    DBG_T(8);
 }
 
 // contiguous copy of the permuted batch (one launch per repeat): minibatch k is then rows
@@ -515,18 +488,6 @@ __device__ __forceinline__ float4 wg_reduced4(const float* red, int m, int n4) {
     return s4;
 }
 
-// Adam hyper-parameters of one optimiser step (torch.optim.Adam scalars, python doubles -> f32)
-struct AdamStep {
-    float w1, b2, w2, bc2s, eps, neg_step;
-};
-
-__device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, const AdamStep& a) {
-    m = m + a.w1 * (g - m);                 // exp_avg.lerp_(grad, 1 - beta1)
-    v = v * a.b2 + (a.w2 * g) * g;          // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
-    const float denom = sqrtf(v) / a.bc2s + a.eps;
-    return p + (a.neg_step * m) / denom;    // param.addcdiv_(exp_avg, denom, value=-step_size)
-}
-
 // Device-wide barrier for co-resident grids (cooperative launch): monotonically increasing ticket
 // counter, one arrival per CTA, spin on an acquire load.
 __device__ __forceinline__ void grid_barrier(unsigned long long* counter, unsigned long long target) {
@@ -599,15 +560,11 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
     pdl_wait();            // dz1 / dz2 / dout of this minibatch are complete
     pdl_trigger();
     float gscale = 1.0f;   // clip coefficient (FUSED)
-    const long long t_start = clock64();
-    (void)t_start;
     auto finish = [&]() {  // norm contribution (+ barrier and clip scale when fused)
-        if (FUSED && tid == 0) { const int c = bx + 40 * net; DBG_CTA(c, clock64() - t_start); }
         const float tot = block_sum_256(sq, s_red);
         if (tid == 0 && tot != 0.f && u.world <= 1) atomicAdd(u.norm_sq, tot);   // DP: the norm of the REDUCED gradient is taken later
         if (FUSED) {
             grid_barrier(bar, bar_target);
-            if (tid == 0) { const int c = bx + 40 * net; DBG_CTA(256 + c, clock64() - t_start); }
             const float nsq = __ldcg(u.norm_sq);
             if (u.max_grad_norm > 0.f) gscale = fminf(u.max_grad_norm / (sqrtf(nsq) + 1e-6f), 1.0f);
             if (bx == 0 && net == 0 && tid == 0 && u.stats && slot >= 0)
@@ -615,6 +572,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
         }
     };
     const long long pbase = u.net_off[net];
+    const NetLayout L = ppo_layout(u, net, H);
     if (bx < NT) {
         // ---- dW2t[k][o] = sum_r h1[r][k] * dz2[r][o] : 32 x 64 tile, 2 x 4 per thread (FFMA issue is the
         // bound on this chip, so the tiles are sized to spread over ~all SMs) ---------------------------
@@ -627,7 +585,6 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
 #pragma unroll
             for (int nt = 0; nt < 8; ++nt) { c[mt][nt][0] = c[mt][nt][1] = c[mt][nt][2] = c[mt][nt][3] = 0.f; }
         float bpart = 0.f;                                  // db2: thread (o = tid % 64, row group tid / 64)
-        DBG_W(10);
         pipeline([&](int ch, int buf) { stage(ch, buf, nv.s_h1, H, k0, WG_TKT, nv.s_dz2, H, o0, WG_T); },
                  [&](int buf) {
                      wg_mma_chunk<2, 8>(sLp(buf), sGp(buf), c);
@@ -637,7 +594,6 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
                          for (int rr = tid / WG_T; rr < WG_RC; rr += WG_TPB / WG_T) bpart += G[(size_t)rr * WG_LD];
                      }
                  });
-        DBG_W(11);
         float* red = smem;                                  // staging is dead: cross-warp reduction buffer
         float* bred = smem + 2 * WG_NST * WG_CHUNK + 80 * WG_T;      // [4][WG_T] bias partials
         wg_store_partial<2, 8>(red, c);
@@ -654,9 +610,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
 #pragma unroll
         for (int i = 0; i < 2; ++i) sq += acc[i][0] * acc[i][0] + acc[i][1] * acc[i][1] + acc[i][2] * acc[i][2] + acc[i][3] * acc[i][3];
         if (do_bias && tid < WG_T) sq += bsum * bsum;
-        DBG_W(12);
         finish();
-        DBG_W(13);
         if (!FUSED) {
 #pragma unroll
             for (int i = 0; i < 2; ++i)
@@ -664,7 +618,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
                     make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
             if (do_bias && tid < WG_T) nv.g_b2[o0 + tid] = bsum;
         } else {
-            const long long w2s = pbase + (long long)u.D * H + H;
+            const long long w2s = pbase + L.w2;
             float np[2][4];
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
@@ -684,7 +638,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
             for (int j = 0; j < 4; ++j)
                 *reinterpret_cast<float2*>(mir + (size_t)(o0 + 4 * to + j) * H + k0 + 2 * tk) = make_float2(np[0][j], np[1][j]);
             if (do_bias && tid < WG_T) {
-                const long long idx = w2s + (long long)H * H + o0 + tid;
+                const long long idx = pbase + L.b2 + o0 + tid;
                 float m = u.adam_m[idx], v = u.adam_v[idx];
                 u.theta[idx] = adam_one(u.theta[idx], bsum * gscale, m, v, ad);
                 u.adam_m[idx] = m; u.adam_v[idx] = v;
@@ -751,7 +705,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
             const float g = fin[(size_t)d * WG_T + o];
             if (!FUSED) nv.g_w1t[(size_t)d * H + o0 + o] = g;
             else {
-                const long long idx = pbase + (long long)d * H + o0 + o;
+                const long long idx = pbase + L.w1 + (long long)d * H + o0 + o;
                 float m = u.adam_m[idx], v = u.adam_v[idx];
                 u.theta[idx] = adam_one(u.theta[idx], g * gscale, m, v, ad);
                 u.adam_m[idx] = m; u.adam_v[idx] = v;
@@ -761,7 +715,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
             const float g = fin[(size_t)D * WG_T + o];
             if (!FUSED) nv.g_b1[o0 + o] = g;
             else {
-                const long long idx = pbase + (long long)D * H + o0 + o;
+                const long long idx = pbase + L.b1 + o0 + o;
                 float m = u.adam_m[idx], v = u.adam_v[idx];
                 u.theta[idx] = adam_one(u.theta[idx], g * gscale, m, v, ad);
                 u.adam_m[idx] = m; u.adam_v[idx] = v;
@@ -815,7 +769,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
             if (j < out) {
                 if (!FUSED) nv.g_w3t[(size_t)(k0 + k) * out + j] = acc[q];
                 else {
-                    const long long idx = pbase + (long long)u.D * H + H + (long long)H * H + H + (long long)(k0 + k) * out + j;
+                    const long long idx = pbase + L.w3 + (long long)(k0 + k) * out + j;
                     float m = u.adam_m[idx], v = u.adam_v[idx];
                     u.theta[idx] = adam_one(u.theta[idx], acc[q] * gscale, m, v, ad);
                     u.adam_m[idx] = m; u.adam_v[idx] = v;
@@ -823,8 +777,7 @@ __device__ __forceinline__ void ppo_wgrad_role(const fsrl_ppo_update_t& u, int m
             }
         }
         if (own_b3 || own_ls) {
-            const long long b3s = pbase + (long long)u.D * H + H + (long long)H * H + H + (long long)H * out;
-            const long long idx = own_b3 ? b3s + tid : b3s + out + (tid - A);
+            const long long idx = own_b3 ? pbase + L.b3 + tid : pbase + L.extra + (tid - A);
             if (!FUSED) { if (own_b3) nv.g_b3[tid] = csum; else nv.g_log_sigma[tid - A] = csum; }
             else {
                 float m = u.adam_m[idx], v = u.adam_v[idx];
@@ -839,11 +792,7 @@ template <int H>
 __global__ void __launch_bounds__(WG_TPB)
 ppo_wgrad_kernel(const fsrl_ppo_update_t u, int mb_off, int B) {
     extern __shared__ __align__(16) float smem[];
-    AdamStep ad = {};
-    const long long t0 = clock64();
-    (void)t0;
-    ppo_wgrad_role<H, false>(u, mb_off, B, blockIdx.x, blockIdx.y, smem, ad, nullptr, 0ULL, -1);
-    if (threadIdx.x == 0) DBG_CTA(blockIdx.x + gridDim.x * blockIdx.y, clock64() - t0);
+    ppo_wgrad_role<H, false>(u, mb_off, B, blockIdx.x, blockIdx.y, smem, AdamStep{}, nullptr, 0ULL, -1);
 }
 
 // weight gradients + clip_grad_norm_ + Adam in one launch with a grid barrier (single-GPU path)
@@ -858,17 +807,8 @@ ppo_wgrad_adam_kernel(const fsrl_ppo_update_t u, int mb_off, int B, AdamStep ad,
 // ------------------------------------------------------------------------------------------
 // Phase C: clip_grad_norm_ + Adam (torch.optim.Adam single-tensor arithmetic order)
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ float adam_one_s(float p, float g, float& m, float& v, float w1, float b2,
-                                            float w2, float bc2s, float eps, float neg_step) {
-    m = m + w1 * (g - m);                 // exp_avg.lerp_(grad, 1 - beta1)
-    v = v * b2 + (w2 * g) * g;            // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
-    const float denom = sqrtf(v) / bc2s + eps;
-    return p + (neg_step * m) / denom;    // param.addcdiv_(exp_avg, denom, value=-step_size)
-}
-
 __global__ void __launch_bounds__(256)
-adam_kernel(const fsrl_ppo_update_t u, float w1, float b2, float w2, float bc2s, float eps,
-            float neg_step, int slot, int n_plain_blocks) {
+adam_kernel(const fsrl_ppo_update_t u, const AdamStep ad, int slot, int n_plain_blocks) {
     __shared__ float tile[32][33];
     __shared__ float nred[8];
     pdl_wait();                        // gradients / norm partials of this step are complete
@@ -899,25 +839,27 @@ adam_kernel(const fsrl_ppo_update_t u, float w1, float b2, float w2, float bc2s,
         long long i = -1;
         for (int n = 0; n < u.n_nets; ++n) {
             const long long size = ((n + 1 < u.n_nets) ? u.net_off[n + 1] : u.n_params) - u.net_off[n];
-            const long long pre = (long long)u.D * H + H, post = size - pre - (long long)H * H;
+            const NetLayout L = ppo_layout(u, n, H);
+            const long long pre = L.w2, post = size - L.b2;
             if (cc < pre) { i = u.net_off[n] + cc; break; }
             cc -= pre;
-            if (cc < post) { i = u.net_off[n] + pre + (long long)H * H + cc; break; }
+            if (cc < post) { i = u.net_off[n] + L.b2 + cc; break; }
             cc -= post;
         }
         if (i < 0) return;
         float m = u.adam_m[i], v = u.adam_v[i];
         const float g = (u.mask && u.mask[i] == 0) ? 0.f : u.grad[i] * scale;
         if (u.mask && u.mask[i] == 0) return;
-        u.theta[i] = adam_one_s(u.theta[i], g, m, v, w1, b2, w2, bc2s, eps, neg_step);
+        u.theta[i] = adam_one(u.theta[i], g, m, v, ad);
         u.adam_m[i] = m; u.adam_v[i] = v;
     } else {
         // W2 tiles: 32 x 32, update canonical W2t[k][o] and its mirror W2n[o][k]
         const int tpn = (H / 32) * (H / 32);
         const int t = blockIdx.x - n_plain_blocks;
-        const int n = t / tpn, tt = t % tpn;
-        const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
-        const long long base = u.net_off[n] + (long long)u.D * H + H;
+        const int n = t / tpn;
+        int k0, o0;
+        w2_tile_origin(t % tpn, H, k0, o0);
+        const long long base = u.net_off[n] + ppo_layout(u, n, H).w2;
         const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
         const bool frozen = u.mask && u.mask[base] == 0;
 #pragma unroll
@@ -927,18 +869,12 @@ adam_kernel(const fsrl_ppo_update_t u, float w1, float b2, float w2, float bc2s,
             float p = u.theta[i];
             if (!frozen) {
                 float m = u.adam_m[i], v = u.adam_v[i];
-                p = adam_one_s(p, u.grad[i] * scale, m, v, w1, b2, w2, bc2s, eps, neg_step);
+                p = adam_one(p, u.grad[i] * scale, m, v, ad);
                 u.theta[i] = p; u.adam_m[i] = m; u.adam_v[i] = v;
             }
             tile[kk][lx] = p;
         }
-        __syncthreads();
-        float* mir = u.w2n + (size_t)n * H * H;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int oo = ly + 8 * q;
-            mir[(size_t)(o0 + oo) * H + k0 + lx] = tile[lx][oo];
-        }
+        w2_tile_store_mirror(tile, u.w2n + (size_t)n * H * H, H, k0, o0);
     }
 }
 
@@ -1149,11 +1085,10 @@ static int ppo_launch_minibatch(const fsrl_ppo_update_t& u, int mb_off, int B, i
     // torch.optim.Adam scalars (python doubles -> f32 at the op)
     const double b1 = u.beta1, b2 = u.beta2;
     const double bc1 = 1.0 - pow(b1, (double)adam_t), bc2 = 1.0 - pow(b2, (double)adam_t);
-    const float neg_step = (float)(-(u.lr / bc1));
-    const float bc2s = (float)sqrt(bc2);
+    const AdamStep ad = {(float)(1.0 - b1), (float)b2, (float)(1.0 - b2), (float)sqrt(bc2), (float)u.adam_eps,
+                         (float)(-(u.lr / bc1))};
     if (u.world <= 1 && fuse_ok == 1 && u.barrier != nullptr && u.mask == nullptr) {
         // single GPU: gradients never leave the registers -- tiles -> norm -> barrier -> clip + Adam
-        AdamStep ad = {(float)(1.0 - b1), (float)b2, (float)(1.0 - b2), bc2s, (float)u.adam_eps, neg_step};
         unsigned long long target = (unsigned long long)(bar_count + 1) * gB.x * gB.y;
         // Ordinary (not cooperative) launch: measured 4.6 % faster per cycle.  The grid barrier is still
         // safe: fuse_ok guarantees grid <= SMs x CTAs/SM, every CTA of the grid becomes resident without
@@ -1185,24 +1120,18 @@ static int ppo_launch_minibatch(const fsrl_ppo_update_t& u, int mb_off, int B, i
     }
     const int n_plain = adam_plain_blocks(u, H);
     const int n_tiles = u.n_nets * (H / 32) * (H / 32);
-    FSRL_CUDA(launch_chain(adam_kernel, dim3(n_plain + n_tiles), dim3(256), (size_t)0, s, false, u, (float)(1.0 - b1),
-                           (float)b2, (float)(1.0 - b2), bc2s, (float)u.adam_eps, neg_step, slot, n_plain));
+    FSRL_CUDA(launch_chain(adam_kernel, dim3(n_plain + n_tiles), dim3(256), (size_t)0, s, false, u, ad, slot, n_plain));
     return FSRL_OK;
 }
 
-__global__ void mirror_w2_kernel(const fsrl_ppo_update_t u) {
-    // w2n[n][o][k] = w2t[n][k][o]  (initial sync of the mirror, 32x32 tiles)
-    __shared__ float tile[32][33];
-    const int H = u.H;
-    const int tpn = (H / 32) * (H / 32);
-    const int n = blockIdx.x / tpn, tt = blockIdx.x % tpn;
-    const int k0 = (tt / (H / 32)) * 32, o0 = (tt % (H / 32)) * 32;
-    const float* src = u.theta + u.net_off[n] + (long long)u.D * H + H;
-    const int lx = threadIdx.x % 32, ly = threadIdx.x / 32;
-    for (int q = 0; q < 4; ++q) tile[ly + 8 * q][lx] = src[(size_t)(k0 + ly + 8 * q) * H + o0 + lx];
-    __syncthreads();
-    float* mir = u.w2n + (size_t)n * H * H;
-    for (int q = 0; q < 4; ++q) mir[(size_t)(o0 + ly + 8 * q) * H + k0 + lx] = tile[lx][ly + 8 * q];
+// w2n[n] <- transpose of every net's W2 block, one launch
+static int sync_mirror(const fsrl_ppo_update_t& u, cudaStream_t s) {
+    W2Mirrors m = {};
+    for (int n = 0; n < u.n_nets; ++n) {
+        m.w2t[n] = u.theta + u.net_off[n] + ppo_layout(u, n, u.H).w2;
+        m.w2n[n] = u.w2n + (size_t)n * u.H * u.H;
+    }
+    return w2_mirror(m, u.n_nets, u.H, s);
 }
 
 }  // namespace fsrl
@@ -1233,17 +1162,14 @@ extern "C" size_t fsrl_ppo_persist_ws_floats(int n_nets, int D, int H) { return 
 extern "C" size_t fsrl_ppo_persist_p2p_floats(int n_nets) { return ppo_persist_p2p_floats(n_nets); }
 
 extern "C" int fsrl_ppo_persist_active(const fsrl_ppo_update_t* u, long long n_total, int batch_size) {
-    if (!u || u->persist_off || getenv("FSRL_PPO_NO_PERSIST")) return 0;
+    if (!u || u->persist_off) return 0;
     return ppo_persist_supported(*u, n_total, batch_size) ? 1 : 0;
 }
 
 extern "C" int fsrl_ppo_sync_mirror(const fsrl_ppo_update_t* u, void* stream) {
     int rc = check_update(u);
     if (rc) return rc;
-    const int H = u->H;
-    mirror_w2_kernel<<<u->n_nets * (H / 32) * (H / 32), 256, 0, static_cast<cudaStream_t>(stream)>>>(*u);
-    FSRL_LAUNCH_CHECK();
-    return FSRL_OK;
+    return sync_mirror(*u, static_cast<cudaStream_t>(stream));
 }
 
 // One repeat of PPOLagrangian.learn's inner loop (ppo_lag.py:223-247): every minibatch of
@@ -1297,14 +1223,14 @@ extern "C" int fsrl_ppo_lag_epoch(const fsrl_ppo_update_t* u, long long n_total,
         ppo_adv_stats_kernel<<<n_mb, 256, 0, s>>>(*u, n_total, n_mb);
         FSRL_LAUNCH_CHECK();
     }
-    if (!u->persist_off && !getenv("FSRL_PPO_NO_PERSIST") && ppo_persist_supported(*u, n_total, batch_size)) {
+    if (!u->persist_off && ppo_persist_supported(*u, n_total, batch_size)) {
         // one persistent launch runs every minibatch of the repeat (csrc/ppo_persist.cu); the out-major
         // mirror of W2 that the three-launch chain reads is refreshed afterwards
         const int n_mb = (int)(n_total / batch_size);
         int rcp = ppo_persist_run(*u, n_mb, stats_slot0, adam_t0, s);
         if (rcp) return rcp;
-        mirror_w2_kernel<<<u->n_nets * (u->H / 32) * (u->H / 32), 256, 0, s>>>(*u);
-        FSRL_LAUNCH_CHECK();
+        rcp = sync_mirror(*u, s);
+        if (rcp) return rcp;
         if (n_minibatches) *n_minibatches = n_mb;
         return FSRL_OK;
     }
@@ -1326,68 +1252,5 @@ extern "C" int fsrl_ppo_lag_epoch(const fsrl_ppo_update_t* u, long long n_total,
         if (last) break;
     }
     if (n_minibatches) *n_minibatches = count;
-    return FSRL_OK;
-}
-
-// Measurement aid for bench.py's roofline object: average duration of each phase kernel over
-// `iters` back-to-back launches on one minibatch of u->perm (CUDA events on `stream`).  The
-// Adam phase is launched with lr = 0 so that the weights are not disturbed.
-template <int H>
-static int ppo_time_phases(const fsrl_ppo_update_t& u0, int B, int iters, float* ms, cudaStream_t s) {
-    using TT = MlpTile<H>;
-    fsrl_ppo_update_t u = u0;
-    const size_t smemF = sizeof(float) * ((size_t)TT::R * TT::in_pad(u.D) + (size_t)TT::R * TT::LDA + slab_buf_floats<H>());
-    const size_t smemB = sizeof(float) * (2 * (size_t)TT::R * TT::LDA + slab_buf_floats<H>() + (size_t)H * (u.actor_out > 1 ? u.actor_out : 1) + (size_t)TT::R * DOUT_LD);
-    FSRL_CUDA(cudaFuncSetAttribute(ppo_fwd_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemF));
-    FSRL_CUDA(cudaFuncSetAttribute(ppo_bwd_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemB));
-    cudaEvent_t e[5];
-    for (int i = 0; i < 5; ++i) FSRL_CUDA(cudaEventCreate(&e[i]));
-    const dim3 gA((B + TT::R - 1) / TT::R, H / SLAB_NS, u.n_nets);
-    constexpr int NTT = H / WG_T;
-    const dim3 gB((H / WG_TKT) * NTT + 2 * NTT, u.n_nets);
-    const size_t smemW = sizeof(float) * WG_SMEM_FLOATS;
-    FSRL_CUDA(cudaFuncSetAttribute(ppo_wgrad_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemW));
-    const int n_plain = adam_plain_blocks(u, H);
-    const int n_tiles = u.n_nets * (H / 32) * (H / 32);
-    FSRL_CUDA(cudaEventRecord(e[0], s));
-    for (int i = 0; i < iters; ++i) ppo_fwd_kernel<H><<<gA, MLP_TPB, smemF, s>>>(u, 0, B);
-    FSRL_CUDA(cudaEventRecord(e[1], s));
-    for (int i = 0; i < iters; ++i) ppo_bwd_kernel<H><<<gA, MLP_TPB, smemB, s>>>(u, 0, B, 0);
-    FSRL_CUDA(cudaEventRecord(e[2], s));
-    for (int i = 0; i < iters; ++i) ppo_wgrad_kernel<H><<<gB, WG_TPB, smemW, s>>>(u, 0, B);
-    FSRL_CUDA(cudaEventRecord(e[3], s));
-    for (int i = 0; i < iters; ++i)
-        adam_kernel<<<n_plain + n_tiles, 256, 0, s>>>(u, 0.1f, 0.999f, 0.001f, 1.0f, 1e-8f, 0.0f, -1, n_plain);
-    FSRL_CUDA(cudaEventRecord(e[4], s));
-    FSRL_CUDA(cudaEventSynchronize(e[4]));
-    for (int i = 0; i < 4; ++i) {
-        float t = 0.f;
-        FSRL_CUDA(cudaEventElapsedTime(&t, e[i], e[i + 1]));
-        ms[i] = t / (float)iters;
-    }
-    for (int i = 0; i < 5; ++i) cudaEventDestroy(e[i]);
-    FSRL_LAUNCH_CHECK();
-    return FSRL_OK;
-}
-
-extern "C" int fsrl_ppo_phase_times(const fsrl_ppo_update_t* u, int B, int iters, float* ms_out, void* stream) {
-    int rc = check_update(u);
-    if (rc) return rc;
-    FSRL_REQUIRE(ms_out && iters > 0 && B > 1 && B <= u->bmax, "fsrl_ppo_phase_times: bad arguments");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    switch (u->H) {
-        case 64: return ppo_time_phases<64>(*u, B, iters, ms_out, s);
-        case 128: return ppo_time_phases<128>(*u, B, iters, ms_out, s);
-        case 256: return ppo_time_phases<256>(*u, B, iters, ms_out, s);
-        default: return ppo_time_phases<512>(*u, B, iters, ms_out, s);
-    }
-}
-
-extern "C" int fsrl_debug_clocks(long long* out32) {
-    FSRL_CUDA(cudaMemcpyFromSymbol(out32, fsrl::g_dbg_clock, sizeof(long long) * 32));
-    return FSRL_OK;
-}
-extern "C" int fsrl_debug_cta_cycles(long long* out512) {
-    FSRL_CUDA(cudaMemcpyFromSymbol(out512, fsrl::g_dbg_cta, sizeof(long long) * 512));
     return FSRL_OK;
 }

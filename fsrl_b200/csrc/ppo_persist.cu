@@ -33,6 +33,7 @@
 // gradients itself over peer memory (dp_* functions below: tagged + hashed 16-byte packets pushed into the peers' buffers).
 // DESIGN.md 3a / 6 hold the measurements behind these choices.
 #include "ppo_persist.cuh"
+#include "arena.cuh"
 #include "umma.cuh"
 #include <cstdlib>
 #include <cmath>
@@ -114,11 +115,12 @@ constexpr int DBG_N = 48;
 #define STAMP(i) do { if (P.dbg && t == P.dbg_step) P.dbg[(size_t)blockIdx.x * DBG_N + (i)] = clock64(); } while (0)
 
 struct AdamS { float w1, b2, w2, rbc2s, eps, neg_step; };
-// torch.optim.Adam's single-tensor update.  The moments are the exact fp32 expressions; the parameter step
-// p += step * m / (sqrt(v) / sqrt(bc2) + eps) uses the SFU reciprocal square root / reciprocal (about 2 ulp each,
-// i.e. ~1e-10 absolute on a step of <= lr) instead of IEEE sqrt and division, whose slow-path calls serialise the
-// 32 elements a lane owns (measured: 19k cycles per step for the 64 x 64 tile with IEEE arithmetic).
-__device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, const AdamS& a) {
+// torch.optim.Adam's single-tensor update, approximate variant of arena.cuh's adam_one.  The moments are the exact
+// fp32 expressions; the parameter step p += step * m / (sqrt(v) / sqrt(bc2) + eps) uses the SFU reciprocal square
+// root / reciprocal (about 2 ulp each, i.e. ~1e-10 absolute on a step of <= lr) instead of IEEE sqrt and division,
+// whose slow-path calls serialise the 32 elements a lane owns (measured: 19k cycles per step for the 64 x 64 tile
+// with IEEE arithmetic).
+__device__ __forceinline__ float adam_one_approx(float p, float g, float& m, float& v, const AdamS& a) {
     m = m + a.w1 * (g - m);                 // exp_avg.lerp_(grad, 1 - beta1)
     v = v * a.b2 + (a.w2 * g) * g;          // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
     const float sq = v > 0.f ? v * rsqrtf(v) : 0.f;
@@ -561,8 +563,9 @@ __global__ void __launch_bounds__(TPB, 1) ppo_persist_kernel(const Args P) {
 
     // parameter offsets of this network inside the flat arena
     const long long pbase = u.net_off[net];
-    const long long o_w1 = pbase, o_b1 = o_w1 + (long long)D * H, o_w2 = o_b1 + H, o_b2 = o_w2 + (long long)H * H,
-                    o_w3 = o_b2 + H, o_b3 = o_w3 + (long long)H * out, o_ls = o_b3 + out;
+    const NetLayout L(D, H, out, (net == 0 && u.head_indep) ? A : 0);
+    const long long o_w1 = pbase + L.w1, o_b1 = pbase + L.b1, o_w2 = pbase + L.w2, o_b2 = pbase + L.b2,
+                    o_w3 = pbase + L.w3, o_b3 = pbase + L.b3, o_ls = pbase + L.extra;
 
     if (warp == 0) {
         // ============================ bulk-copy producer ==========================================
@@ -1242,7 +1245,7 @@ __global__ void __launch_bounds__(TPB, 1) ppo_persist_kernel(const Args P) {
             // ---- clip + Adam: replicated small slices, then the owned W2 tile (tensor memory) --------------------
             for (int i = et; i < sm.n; i += NEPI) {
                 float m = sp_m[i], v = sp_v[i];
-                sp_p[i] = adam_one(sp_p[i], sp_g[i] * gscale, m, v, ad);
+                sp_p[i] = adam_one_approx(sp_p[i], sp_g[i] * gscale, m, v, ad);
                 sp_m[i] = m; sp_v[i] = v;
             }
             if (et == 0) STAMP(25);
@@ -1252,7 +1255,7 @@ __global__ void __launch_bounds__(TPB, 1) ppo_persist_kernel(const Args P) {
                 else acc_ld_split<C2>(tm_lane, lane, C2 * wq, 32 + C2 * wq, g);
                 tmem_ldn<C2>(tm_lane + TM_P + C2 * wq, pv); tmem_ldn<C2>(tm_lane + TM_M + C2 * wq, mv); tmem_ldn<C2>(tm_lane + TM_V + C2 * wq, vv);
 #pragma unroll
-                for (int j = 0; j < C2; ++j) pv[j] = adam_one(pv[j], g[j] * gscale, mv[j], vv[j], ad);
+                for (int j = 0; j < C2; ++j) pv[j] = adam_one_approx(pv[j], g[j] * gscale, mv[j], vv[j], ad);
                 tmem_stn<C2>(tm_lane + TM_P + C2 * wq, pv); tmem_stn<C2>(tm_lane + TM_M + C2 * wq, mv); tmem_stn<C2>(tm_lane + TM_V + C2 * wq, vv);
             }
             tc_fence_before();
@@ -1362,7 +1365,7 @@ int ppo_persist_run(const fsrl_ppo_update_t& ug, int n_mb, int stats_slot0, long
     }
     bool cluster = !getenv("FSRL_PPO_NO_CLUSTER") && pp::smem_bytes(ug.D, true) + 8192 <= (size_t)smem_optin;
     size_t smem = pp::smem_bytes(ug.D, cluster);
-    const bool dp = ug.world > 1 || getenv("FSRL_PPO_FORCE_DP_KERNEL") != nullptr;   // (the env switch: code-generation experiments)
+    const bool dp = ug.world > 1;
     void (*kern)(const pp::Args) = dp ? pp::ppo_persist_kernel<true> : pp::ppo_persist_kernel<false>;
     static size_t set[2] = {0, 0};
     if (smem > set[dp]) {

@@ -213,14 +213,6 @@ int fsrl_ppo_sync_mirror(const fsrl_ppo_update_t* u, void* stream);
  * statistics go to stats[stats_slot0 + i]; *n_minibatches (host) receives the count */
 int fsrl_ppo_lag_epoch(const fsrl_ppo_update_t* u, long long n_total, int batch_size,
                        int stats_slot0, long long adam_t0, int* n_minibatches, void* stream);
-/* measurement aid (bench.py roofline): mean duration [ms] of the four phase kernels (fwd, bwd,
- * wgrad, adam) over
- * `iters` launches on the first B rows of u->perm; weights are left untouched (lr = 0) */
-/* tuning aid: clock64() stamps taken by CTA (0,0) at the phase boundaries of the last
- * ppo_fwdbwd launch (host array of 16) */
-int fsrl_debug_clocks(long long* out32);   /* 32 stamps; only written by -DFSRL_DEBUG_CLOCKS builds */
-int fsrl_debug_cta_cycles(long long* out512); /* per-CTA cycle counts of the last ppo_wgrad launch */
-int fsrl_ppo_phase_times(const fsrl_ppo_update_t* u, int B, int iters, float* ms_out, void* stream);
 
 /* ---- a6: batched critic / actor forward ---------------------------------------------------
  * y[r][:] = net(x[idx ? idx[r] : r][:]) for r < n_rows.  Replaces the chunked no_grad

@@ -55,49 +55,12 @@ def bench_gae(envs, T):
                       "alg_bytes": alg_bytes, "GBps": gbs, "frac_of_%s_hbm" % how: gbs / pk["hbm_gbs"]}))
 
 
-def bench_ppo(iters):
-    import bench
-    agent, trainer, col, buf, T = bench.build("cuda:0", 0)
-    print(json.dumps({"phase_ms(fwd,bwd,wgrad,adam)": bench.phase_times(agent, col, buf, iters=iters)}))
-    import ctypes
-    from fsrl_b200 import _lib
-    ck = (ctypes.c_longlong * 32)()
-    _lib.check(_lib.lib.fsrl_debug_clocks(ck))
-    c = list(ck)
-    print("ppo_bwd CTA(0,0,0) cycles [loads, advstats, sync, head, lossgrad, stats, dz2, wait_slab, slab_gemm]:",
-          [c[i + 1] - c[i] for i in range(8)], "total", c[8] - c[0])
-    print("ppo_fwd CTA(0,0,0) cycles [obs load, (pdl wait), slab issue+sync, layer1, wait_slab, slab_gemm]:",
-          [c[i + 1] - c[i] for i in range(16, 22)], "total", c[22] - c[16])
-    cc = (ctypes.c_longlong * 512)()
-    _lib.check(_lib.lib.fsrl_debug_cta_cycles(cc))
-    cc = list(cc)[:120]
-    print("wgrad per-CTA cycles net0 roles:", cc[:40])
-    print("wgrad tile CTA cycles [stage0 issue, chunk loop, finish]:", [c[11] - c[10], c[12] - c[11], c[13] - c[12]])
-
-
-def bench_fused():
-    import bench, ctypes
-    from fsrl_b200 import _lib
-    agent, trainer, col, buf, T = bench.build("cuda:0", 0)
-    bench.one_cycle(trainer)
-    torch.cuda.synchronize()
-    cc = (ctypes.c_longlong * 512)()
-    _lib.check(_lib.lib.fsrl_debug_cta_cycles(cc))
-    cc = list(cc)
-    print("fused wgrad: cycles to end of role compute, net0 roles [32 tiles | 4 L1 | 4 L3]:", cc[:40])
-    print("fused wgrad: cycles to barrier exit, net0:", cc[256:296])
-
-
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("what")
+    ap.add_argument("what", choices=["gae"])
     ap.add_argument("--envs", type=int, default=2048)
     ap.add_argument("--T", type=int, default=300)
     a = ap.parse_args()
-    if a.what == "fused":
-        bench_fused()
-    if a.what == "ppo":
-        bench_ppo(a.T if a.T != 300 else 50)
     if a.what == "gae":
         bench_gae(a.envs, a.T)
         bench_gae(a.envs * 16, a.T)
